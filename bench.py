@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """Benchmark of the torchcde_b200 hot path against BASELINE.json's metric.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one fused fixed-step solve ``cdeint(CubicSpline(hermite coeffs), linear func, z0,
 t=[0, L-1], method='rk4', options={'step_size': 1})`` over one synthetic batch at BASELINE
 config 3: batch 65536 per GPU, length 256, 8 input channels, 32 hidden channels, fp32.
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for what every key means.
+
+``--dump-outputs DIR`` writes what the last timed step returned on rank 0 -- the whole
+``cdeint`` output, (65536, 2, 32) float32, 16 MB -- as ``DIR/cdeint_out.npy``.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 
 Timing rules: inputs resident in HBM for ``value`` (CUDA events, max over ranks, barrier +
 synchronize both sides); the coefficient tensor is 2.1 GB per GPU, far larger than the 126 MB
@@ -25,6 +29,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the tree may be read-only: leave no __pycache__ behind in it
 
 import torch  # noqa: E402
 
@@ -359,6 +364,10 @@ def run_gpu_arm(args):
         if rank != 0:
             clocks = None
         assert bool(torch.isfinite(holder["out"]).all())
+        if args.dump_outputs and rank == 0:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "cdeint_out.npy"), holder["out"].float().cpu().numpy())
 
         note("device-resident: {:.3f} ms per solve".format(ms / args.steps))
         # ---- end to end from pinned host buffers (copies inside the timed region) ------------
@@ -623,7 +632,11 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--variant", type=int, default=None, help="solve kernel: 1 = CUDA-core, 2 = tcgen05 (default: the library's choice)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step (rank 0) as DIR/cdeint_out.npy, float32")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the output of the CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         run_reference_arm(args)

@@ -1,6 +1,6 @@
 """Generate tests/golden/*.npz from the LIVE reference -- run in the build container only.
 
-    python -m oracle.make_golden
+    python -m oracle.make_golden [fixture ...]      (default: every fixture in FIXTURES)
 
 Every array under ``ref_*`` keys is an output of the unmodified reference code imported
 from /root/reference (``oracle/reference_loader.py``); the ``in_*`` arrays are the seeded
@@ -239,17 +239,216 @@ def solves(ref):
     return n
 
 
-def main():
+def bit_digest(x):
+    """SHA-256 of a tensor's dtype, shape and values, with every NaN made the same NaN and -0 made +0: two tensors
+    have the same digest exactly when ``conftest.same`` calls them equal (up to hash collisions)."""
+    import hashlib
+    x = x.detach().cpu().contiguous()
+    x = torch.where(torch.isnan(x), torch.full_like(x, NAN), x) + 0
+    head = "{}{}".format(x.dtype, tuple(x.shape)).encode()
+    return hashlib.sha256(head + x.numpy().tobytes()).hexdigest()
+
+
+def builders_fresh(ref):
+    """The builders once more on a second seeded set of shapes (4-d batches, a single channel, length 2).  The
+    comparison is bit for bit, so each reference output is stored as its ``bit_digest``: row n of ``ref_digests``
+    holds case n's, in the order of ``ref_names``."""
+    gen = torch.Generator().manual_seed(31337)
+    cases = {}
+    digests = []
+    n = 0
+    for dtype in (torch.float32, torch.float64):
+        for shape in ((4, 11, 3), (2, 2, 5, 2), (6, 2, 1)):
+            x = torch.randn(shape, generator=gen, dtype=torch.float64).to(dtype)
+            t = (torch.rand(shape[-2], generator=gen, dtype=torch.float64) + 0.05).cumsum(0).to(dtype)
+            for frac in (0.0, 0.25, 0.7):
+                xin = x.clone()
+                xin[torch.rand(shape, generator=gen) < frac] = NAN
+                for tt in (None, t):
+                    key = "c{:03d}".format(n)
+                    n += 1
+                    cases[key + "_in_x"] = _np(xin)
+                    if tt is not None:
+                        cases[key + "_in_t"] = _np(tt)
+                    digests.append([bit_digest(out) for out in (
+                        ref.linear_interpolation_coeffs(xin, tt),
+                        ref.hermite_cubic_coefficients_with_backward_differences(xin, tt),
+                        ref.natural_cubic_coeffs(xin, tt), ref.natural_cubic_spline_coeffs(xin, tt),
+                        ref.misc.forward_fill(xin))])
+    cases["ref_names"] = np.array(["linear", "hermite", "natural_v1", "natural_v0", "ffill"])
+    cases["ref_digests"] = np.array(digests)
+    cases["count"] = np.array(n)
+    np.savez_compressed(os.path.join(OUT, "builders_fresh.npz"), **cases)
+    return n
+
+
+def _diff_data(seed, batch=(3,), length=9, channels=2, nan=0.0, irregular=True):
+    gen = torch.Generator().manual_seed(seed)
+    x = torch.randn(*batch, length, channels, generator=gen, dtype=torch.float64)
+    if nan:
+        hole = torch.rand(x.shape, generator=gen) < nan
+        x = x.masked_fill(hole, NAN)
+    t = torch.rand(length, generator=gen, dtype=torch.float64).add(0.2).cumsum(0) if irregular else None
+    return x, t
+
+
+def diff_formulas(ref):
+    """Values and gradients (with respect to the data and the knots) of the reference builders, fp64, with and
+    without missing values, for the torch-operator backward passes of torchcde_b200/_diff.py.  Input ``g*``: data
+    (and knots) with the missing-value pattern ``g*_nan`` on a regular or irregular grid.  Case ``d*``: one builder
+    on input ``d*_group``, its output, a seeded cotangent and the reference's gradients of <cotangent, output> (NaN
+    outputs masked out; an input the output does not depend on gets a gradient of zeros(1))."""
+    cases = {}
+    n = 0
+    groups = 0
+    builders_by_name = {"hermite": ref.hermite_cubic_coefficients_with_backward_differences,
+                        "natural1": ref.natural_cubic_coeffs, "natural0": ref.natural_cubic_spline_coeffs,
+                        "linear_fill": ref.linear_interpolation_coeffs}
+    for nan in (0.0, 0.35):
+        for irregular in (False, True):
+            for seed, batch, length in ((0, (3,), 9), (1, (2, 2), 6), (2, (), 2), (3, (4,), 3)):
+                x, t = _diff_data(seed, batch, length, 2, nan, irregular)
+                if nan:
+                    x[..., 1, :] = NAN if length > 2 else x[..., 1, :]      # a fully missing knot row
+                    if batch:
+                        x[0] = NAN                                             # an all-NaN path
+                        x[-1][..., 0, :] = NAN                                 # leading NaN
+                        x[-1][..., -1, 0] = NAN                                # trailing NaN
+                group = "g{:02d}".format(groups)
+                groups += 1
+                cases[group + "_nan"] = np.array(nan)
+                cases[group + "_in_x"] = _np(x)
+                if t is not None:
+                    cases[group + "_in_t"] = _np(t)
+                names = ["hermite", "natural1", "natural0"] + (["linear_fill", "forward_fill"] if nan else [])
+                for name in names:
+                    key = "d{:03d}".format(n)
+                    n += 1
+                    cases[key + "_fn"] = np.array(name)
+                    cases[key + "_group"] = np.array(group)
+                    if name == "forward_fill":
+                        cases[key + "_ref_out"] = _np(ref.misc.forward_fill(x))
+                        continue
+                    xb = x.clone().requires_grad_(True)
+                    tb = None if t is None else t.clone().requires_grad_(True)
+                    want = builders_by_name[name](xb, tb)
+                    ok = ~torch.isnan(want)
+                    # float32-representable, so that it is stored exactly in half the bytes
+                    cot = (torch.randn(want.shape, generator=torch.Generator().manual_seed(seed)) * ok).double()
+                    cases[key + "_ref_out"] = _np(want)
+                    cases[key + "_in_cot"] = _np(cot.float())
+                    cases[key + "_ref_has_grad"] = np.array(want.requires_grad)
+                    if not want.requires_grad:      # linear coefficients without NaN return their input
+                        continue
+                    ins = [xb] + ([tb] if t is not None else [])
+                    grads = torch.autograd.grad(torch.where(ok, want, torch.zeros_like(want)), ins, cot, allow_unused=True)
+                    for label, g in zip(("x", "t"), grads):
+                        g = torch.zeros(1, dtype=torch.float64) if g is None else torch.nan_to_num(g)
+                        cases[key + "_ref_grad_" + label] = _np(g)
+
+    # rectilinear: a time channel without NaN and no leading NaN
+    x, _ = _diff_data(5, (3,), 7, 3, 0.3, False)
+    x[..., 0] = torch.arange(7, dtype=torch.float64)
+    x[:, 0, :] = 1.0
+    cases["rect_in_x"] = _np(x)
+    cases["rect_ref"] = _np(ref.linear_interpolation_coeffs(x, rectilinear=0))
+
+    # spline evaluation: natural cubic + linear interpolation on irregular knots, queries outside, on and between knots
+    x, t = _diff_data(7, (2, 3), 8, 2, 0.0, True)
+    coeffs = ref.natural_cubic_coeffs(x, t)
+    spline = ref.CubicSpline(coeffs, t)
+    linear = ref.LinearInterpolation(x, t)
+    query = torch.tensor([t[0] - 0.3, t[0], t[2], 0.5 * (t[3] + t[4]), t[-1], t[-1] + 1.0], dtype=torch.float64)
+    cases["ev_in_x"] = _np(x)
+    cases["ev_in_t"] = _np(t)
+    cases["ev_ref_coeffs"] = _np(coeffs)
+    for i, q in enumerate((query, query[3], query.view(2, 3))):
+        key = "ev{}".format(i)
+        cases[key + "_in_query"] = _np(q)
+        cases[key + "_ref_index"] = _np(spline._interpret_t(q)[1])
+        cases[key + "_ref_linear_index"] = _np(linear._interpret_t(q)[1])
+        cases[key + "_ref_cubic_eval"] = _np(spline.evaluate(q))
+        cases[key + "_ref_cubic_deriv"] = _np(spline.derivative(q))
+        cases[key + "_ref_linear_eval"] = _np(linear.evaluate(q))
+        cases[key + "_ref_linear_deriv"] = _np(linear.derivative(q))
+    cases["count"] = np.array(n)
+    np.savez_compressed(os.path.join(OUT, "diff_formulas.npz"), **cases)
+    return n
+
+
+def _oracle_signatory():
+    """A ``signatory`` module whose Logsignature is oracle/logsig_oracle.py (signatory itself is not installed)."""
+    import types
+    from . import logsig_oracle
+
+    mod = types.ModuleType("signatory")
+
+    class Logsignature:
+        def __init__(self, depth):
+            self.depth = depth
+
+        def __call__(self, paths):
+            out = [logsig_oracle.logsignature(p.detach().cpu().double().numpy(), self.depth) for p in paths]
+            return torch.tensor(np.stack(out), dtype=paths.dtype)
+
+    mod.Logsignature = Logsignature
+    mod.logsignature_channels = lambda channels, depth: len(logsig_oracle.lyndon_words(channels, depth))
+    return mod
+
+
+def logsig_windows(ref):
+    """The reference's own log_ode.py (window construction, NaN knots, linear fill, scaling, cumsum) with the oracle
+    standing in for signatory: ``logsig_windows`` and ``logsignature_windows``, fp64."""
+    import sys
+    log_ode = sys.modules[ref.__name__ + ".log_ode"]
+    saved = getattr(log_ode, "signatory", None)
+    log_ode.signatory = _oracle_signatory()
+    cases = {}
+    n = 0
+    try:
+        torch.manual_seed(1)
+        for batch, length, channels, depth, window, irregular, nan in (
+                ((2,), 11, 2, 3, 2.5, False, 0.0), ((3,), 9, 3, 2, 4.0, True, 0.3),
+                ((2, 2), 7, 1, 4, 1.0, False, 0.2), ((1,), 6, 2, 2, 10.0, True, 0.0)):
+            x = torch.randn(*batch, length, channels, dtype=torch.float64)
+            if nan:
+                hole = torch.rand(x.shape) < nan
+                hole[..., 0, :] = False
+                hole[..., -1, :] = False
+                x = x.masked_fill(hole, NAN)
+            t = (torch.rand(length, dtype=torch.float64) + 0.3).cumsum(0) if irregular else None
+            key = "w{:02d}".format(n)
+            n += 1
+            cases[key + "_in_x"] = _np(x)
+            if t is not None:
+                cases[key + "_in_t"] = _np(t)
+            cases[key + "_depth"] = np.array(depth)
+            cases[key + "_window"] = np.array(window)
+            cases[key + "_ref_logsig"] = _np(ref.logsig_windows(x, depth, window, t))
+            values, times = ref.logsignature_windows(x, depth, window, t)
+            cases[key + "_ref_values"] = _np(values)
+            cases[key + "_ref_times"] = _np(times)
+    finally:
+        log_ode.signatory = saved
+    cases["count"] = np.array(n)
+    np.savez_compressed(os.path.join(OUT, "logsig_windows.npz"), **cases)
+    return n
+
+
+FIXTURES = {"builders": builders, "rectilinear": rectilinear, "evaluation": evaluation, "solves": solves,
+            "builders_fresh": builders_fresh, "diff_formulas": diff_formulas, "logsig_windows": logsig_windows}
+
+
+def main(names=None):
     torch.set_num_threads(1)
     os.makedirs(OUT, exist_ok=True)
     ref = reference_loader.load_reference()
-    print("builders   :", builders(ref))
-    print("rectilinear:", rectilinear(ref))
-    print("evaluation :", evaluation(ref))
-    print("solves     :", solves(ref))
+    for name in names or FIXTURES:
+        print("{:15s}: {}".format(name, FIXTURES[name](ref)))
     for name in sorted(os.listdir(OUT)):
         print("  {:20s} {:8d} B".format(name, os.path.getsize(os.path.join(OUT, name))))
 
 
 if __name__ == "__main__":
-    main()
+    import sys
+    main(sys.argv[1:])

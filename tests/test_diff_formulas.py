@@ -1,97 +1,81 @@
 """torchcde_b200/_diff.py (the torch-operator restatements that serve BACKWARD passes of the kernel-backed builders)
-against the live reference: same values and the same gradients with respect to the data and the knots, with and
-without missing values.  CPU, fp64.  Needs the reference tree (/root/reference here, oracle/_ref on the GPU box)."""
+against the reference: same values and the same gradients with respect to the data and the knots, with and without
+missing values.  CPU, fp64.  The reference's values and gradients are tests/golden/diff_formulas.npz
+(oracle/make_golden.py)."""
 import pytest
 import torch
 
-from oracle import reference_loader
+from conftest import Golden
 from torchcde_b200 import _diff
 
-pytestmark = pytest.mark.skipif(not reference_loader.reference_available(), reason="reference tree not present")
+_OURS = {"hermite": _diff.hermite, "natural1": lambda a, b: _diff.natural(a, b, 1),
+         "natural0": lambda a, b: _diff.natural(a, b, 0), "linear_fill": _diff.linear_fill}
 
 
-def _data(seed, batch=(3,), length=9, channels=2, nan=0.0, irregular=True):
-    gen = torch.Generator().manual_seed(seed)
-    x = torch.randn(*batch, length, channels, generator=gen, dtype=torch.float64)
-    if nan:
-        hole = torch.rand(x.shape, generator=gen) < nan
-        x = x.masked_fill(hole, float("nan"))
-    t = torch.rand(length, generator=gen, dtype=torch.float64).add(0.2).cumsum(0) if irregular else None
-    return x, t
-
-
-def _compare(ours, theirs, x, t, seed):
+def _compare(g, k, ours, x, t):
     xa = x.clone().requires_grad_(True)
-    xb = x.clone().requires_grad_(True)
     ta = None if t is None else t.clone().requires_grad_(True)
-    tb = None if t is None else t.clone().requires_grad_(True)
-    got, want = ours(xa, ta), theirs(xb, tb)
+    got, want = ours(xa, ta), g.t(k + "_ref_out")
     assert got.shape == want.shape
     nan_same = torch.isnan(got) == torch.isnan(want)
     assert bool(nan_same.all())
     ok = ~torch.isnan(want)
     assert torch.allclose(got[ok], want[ok], rtol=1e-9, atol=1e-11), float((got[ok] - want[ok]).abs().max())
-    cot = torch.randn(want.shape, generator=torch.Generator().manual_seed(seed), dtype=torch.float64) * ok
-    ins_a = [xa] + ([ta] if t is not None else [])
-    ins_b = [xb] + ([tb] if t is not None else [])
-    if not want.requires_grad:          # e.g. linear coefficients without NaN return their input
+    if not bool(g.z[k + "_ref_has_grad"]):          # e.g. linear coefficients without NaN return their input
         return
+    cot = g.t(k + "_in_cot").double()
+    ins_a = [xa] + ([ta] if t is not None else [])
     ga = torch.autograd.grad(torch.where(ok, got, torch.zeros_like(got)), ins_a, cot, allow_unused=True)
-    gb = torch.autograd.grad(torch.where(ok, want, torch.zeros_like(want)), ins_b, cot, allow_unused=True)
-    for a, b in zip(ga, gb):
+    for a, label in zip(ga, ("x", "t")):
         a = torch.zeros(1, dtype=torch.float64) if a is None else torch.nan_to_num(a)
-        b = torch.zeros(1, dtype=torch.float64) if b is None else torch.nan_to_num(b)
+        b = g.t(k + "_ref_grad_" + label)
         assert torch.allclose(a, b, rtol=1e-7, atol=1e-9), float((a - b).abs().max())
 
 
 @pytest.mark.parametrize("nan", [0.0, 0.35])
 @pytest.mark.parametrize("irregular", [False, True])
 def test_builders_values_and_gradients_match_the_reference(nan, irregular):
-    ref = reference_loader.load_reference()
-    for seed, batch, length in ((0, (3,), 9), (1, (2, 2), 6), (2, (), 2), (3, (4,), 3)):
-        x, t = _data(seed, batch, length, 2, nan, irregular)
-        if nan:
-            x[..., 1, :] = float("nan") if length > 2 else x[..., 1, :]      # a fully missing knot row
-            if batch:
-                x[0] = float("nan")                                           # an all-NaN path
-                x[-1][..., 0, :] = float("nan")                               # leading NaN
-                x[-1][..., -1, 0] = float("nan")                              # trailing NaN
-        _compare(_diff.hermite, ref.hermite_cubic_coefficients_with_backward_differences, x, t, seed)
-        _compare(lambda a, b: _diff.natural(a, b, 1), ref.natural_cubic_coeffs, x, t, seed)
-        _compare(lambda a, b: _diff.natural(a, b, 0), ref.natural_cubic_spline_coeffs, x, t, seed)
-        if nan:
-            _compare(_diff.linear_fill, ref.linear_interpolation_coeffs, x, t, seed)
-            ff = ref.misc.forward_fill(x)
+    g = Golden("diff_formulas")
+    checked = 0
+    for i in range(g.count):
+        k = "d{:03d}".format(i)
+        group = g.s(k + "_group")
+        if g.f(group + "_nan") != nan or g.has(group + "_in_t") != irregular:
+            continue
+        x = g.t(group + "_in_x")
+        t = g.t(group + "_in_t") if irregular else None
+        name = g.s(k + "_fn")
+        if name == "forward_fill":
+            ff = g.t(k + "_ref_out")
             mine = _diff.forward_fill(x)
             assert bool(((ff == mine) | (torch.isnan(ff) & torch.isnan(mine))).all())
+        else:
+            _compare(g, k, _OURS[name], x, t)
+        checked += 1
+    assert checked == (20 if nan else 12)
 
 
 def test_rectilinear_matches_the_reference():
-    ref = reference_loader.load_reference()
-    x, _ = _data(5, (3,), 7, 3, 0.3, False)
-    x[..., 0] = torch.arange(7, dtype=torch.float64)          # the time channel has no NaN
-    x[:, 0, :] = 1.0                                           # no leading NaN
-    want = ref.linear_interpolation_coeffs(x, rectilinear=0)
+    g = Golden("diff_formulas")
+    x = g.t("rect_in_x")
+    want = g.t("rect_ref")
     got = _diff.linear_fill(_diff.rectilinear(x, 0), None)
     assert torch.allclose(got, want)
 
 
 def test_evaluation_formulas_match_the_reference():
-    ref = reference_loader.load_reference()
-    x, t = _data(7, (2, 3), 8, 2, 0.0, True)
-    coeffs = ref.natural_cubic_coeffs(x, t)
-    spline = ref.CubicSpline(coeffs, t)
-    linear = ref.LinearInterpolation(x, t)
-    query = torch.tensor([t[0] - 0.3, t[0], t[2], 0.5 * (t[3] + t[4]), t[-1], t[-1] + 1.0], dtype=torch.float64)
+    g = Golden("diff_formulas")
+    x, t, coeffs = g.t("ev_in_x"), g.t("ev_in_t"), g.t("ev_ref_coeffs")
     c = x.size(-1)
     a, b, two_c, three_d = coeffs[..., :c], coeffs[..., c:2 * c], coeffs[..., 2 * c:3 * c], coeffs[..., 3 * c:]
-    for q in (query, query[3], query.view(2, 3)):
-        frac, index = spline._interpret_t(q)
+    for i in range(3):
+        k = "ev{}".format(i)
+        q = g.t(k + "_in_query")
+        index, lindex = g.t(k + "_ref_index"), g.t(k + "_ref_linear_index")
         for deriv in (False, True):
-            want = spline.derivative(q) if deriv else spline.evaluate(q)
+            want = g.t(k + ("_ref_cubic_deriv" if deriv else "_ref_cubic_eval"))
             got = _diff.cubic_eval(a, b, two_c, three_d, t, q, index, deriv)
             assert torch.allclose(got, want, rtol=1e-12, atol=1e-12)
-            want = linear.derivative(q) if deriv else linear.evaluate(q)
-            _, lindex = linear._interpret_t(q)
+            want = g.t(k + ("_ref_linear_deriv" if deriv else "_ref_linear_eval"))
             got = _diff.linear_eval(x, t, q, lindex, deriv)
             assert torch.allclose(got, want, rtol=1e-12, atol=1e-12)

@@ -1,36 +1,18 @@
 """SURVEY 8(f)4: ``logsig_windows`` / ``logsignature_windows`` on the device.  (1) the kernel against the independent fp64
 oracle; (2) the whole transform against the REFERENCE's own log_ode.py executed on the CPU with the oracle plugged in as
-``signatory`` (so the window construction, NaN knots, linear fill, scaling and cumsum are the reference's code);
-(3) the reference's test_log_ode.py:8-36 with the oracle in signatory's place."""
-import sys
-import types
-
+``signatory`` (so the window construction, NaN knots, linear fill, scaling and cumsum are the reference's code; its
+outputs are tests/golden/logsig_windows.npz, oracle/make_golden.py); (3) the reference's test_log_ode.py:8-36 with the
+oracle in signatory's place."""
 import numpy as np
 import pytest
 import torch
 
 import torchcde_b200 as cde
+from conftest import Golden
 from oracle import logsig_oracle as O
-from oracle import reference_loader
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-
-
-def _fake_signatory():
-    mod = types.ModuleType("signatory")
-
-    class Logsignature:
-        def __init__(self, depth):
-            self.depth = depth
-
-        def __call__(self, paths):
-            out = [O.logsignature(p.detach().cpu().double().numpy(), self.depth) for p in paths]
-            return torch.tensor(np.stack(out), dtype=paths.dtype)
-
-    mod.Logsignature = Logsignature
-    mod.logsignature_channels = lambda channels, depth: len(O.lyndon_words(channels, depth))
-    return mod
 
 
 @pytest.mark.parametrize("dtype,tol", [(torch.float64, 1e-11), (torch.float32, 2e-5)])
@@ -51,27 +33,20 @@ def test_kernel_against_the_oracle(dtype, tol):
         assert float((got - want).abs().max()) <= tol * max(1.0, scale), (channels, depth)
 
 
-@pytest.mark.skipif(not reference_loader.reference_available(), reason="reference tree not present")
-def test_whole_transform_against_the_reference_code_with_the_oracle_as_signatory(monkeypatch):
-    ref = reference_loader.load_reference()
-    log_ode = sys.modules[ref.__name__ + ".log_ode"]
-    monkeypatch.setattr(log_ode, "signatory", _fake_signatory())
-    torch.manual_seed(1)
-    for batch, length, channels, depth, window, irregular, nan in (((2,), 11, 2, 3, 2.5, False, 0.0), ((3,), 9, 3, 2, 4.0, True, 0.3),
-                                                                   ((2, 2), 7, 1, 4, 1.0, False, 0.2), ((1,), 6, 2, 2, 10.0, True, 0.0)):
-        x = torch.randn(*batch, length, channels, dtype=torch.float64)
-        if nan:
-            hole = torch.rand(x.shape) < nan
-            hole[..., 0, :] = False
-            hole[..., -1, :] = False
-            x = x.masked_fill(hole, float("nan"))
-        t = (torch.rand(length, dtype=torch.float64) + 0.3).cumsum(0) if irregular else None
-        want = ref.logsig_windows(x, depth, window, t)
-        got = cde.logsig_windows(x.to(DEV), depth, window, None if t is None else t.to(DEV))
+def test_whole_transform_against_the_reference_code_with_the_oracle_as_signatory():
+    g = Golden("logsig_windows")
+    assert g.count == 4
+    for i in range(g.count):
+        k = "w{:02d}".format(i)
+        x = g.t(k + "_in_x")
+        t = g.t(k + "_in_t").to(DEV) if g.has(k + "_in_t") else None
+        depth, window = int(g.z[k + "_depth"]), g.f(k + "_window")
+        want = g.t(k + "_ref_logsig")
+        got = cde.logsig_windows(x.to(DEV), depth, window, t)
         assert got.shape == want.shape
-        assert torch.allclose(got.cpu(), want, rtol=1e-9, atol=1e-10), (batch, length, channels, depth)
-        want_v, want_t = ref.logsignature_windows(x, depth, window, t)
-        got_v, got_t = cde.logsignature_windows(x.to(DEV), depth, window, None if t is None else t.to(DEV))
+        assert torch.allclose(got.cpu(), want, rtol=1e-9, atol=1e-10), (tuple(x.shape), depth)
+        want_v, want_t = g.t(k + "_ref_values"), g.t(k + "_ref_times")
+        got_v, got_t = cde.logsignature_windows(x.to(DEV), depth, window, t)
         assert torch.allclose(got_v.cpu(), want_v, rtol=1e-9, atol=1e-10) and torch.allclose(got_t.cpu(), want_t)
 
 
